@@ -5,7 +5,7 @@ Metric (BASELINE.json): Mpoints/s fused into a 1024x1024 @ 0.05 m grid, and the 
 fraction of the HBM roofline.  One "step" = one sensor frame through the hot path:
 gem_move (scroll) + gem_add_points (transform + variance + bin + per-cell Kalman fold).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 
 N == 1 : BASELINE configs[1] (HDL-64E-shaped 10 Hz stream, 1024x1024 @ 0.05 m, 1 x B200).
 N  > 1 : launched by torchrun, one rank per GPU: one sensor per rank, the global map tiled
@@ -15,6 +15,9 @@ N  > 1 : launched by torchrun, one rank per GPU: one sensor per rank, the global
          cannot be built here (needs Eigen, SURVEY 0.3), so the reference arm times the CPU
          oracle (oracle/gem_oracle.c, a restatement of the reference semantics) on all host
          threads, kind "port".
+
+--dump-outputs DIR (N == 1) : after the timed steps, writes the map they left behind to DIR/<layer>.npy (see
+         dump_outputs); the inputs depend only on the arguments, so two builds can be compared output for output.
 
 Prints exactly one JSON line on rank 0.
 """
@@ -356,6 +359,21 @@ def cpu_baseline_c1(threads):
     return out
 
 
+DUMP_LAYERS = ("elevation", "variance", "intensity", "color_r", "color_g", "color_b", "lowest")
+DUMP_STATS = ("points_in", "points_binned", "cells_touched", "max_points_per_cell")
+
+
+def dump_outputs(m, out_dir: str) -> None:
+    """What a caller of gem_move + gem_add_points_stream holds after the last timed step: every layer the add path
+    writes (L x L float32 each, colours converted exactly) and that step's stats (float64, DUMP_STATS order)."""
+    os.makedirs(out_dir, exist_ok=True)
+    m.sync()
+    for name in DUMP_LAYERS:
+        np.save(os.path.join(out_dir, name + ".npy"), m.get_layer(name).astype(np.float32))
+    st = m.stats()
+    np.save(os.path.join(out_dir, "stats.npy"), np.array([st[k] for k in DUMP_STATS], np.float64))
+
+
 # ------------------------------------------------------------------------------------------
 def run_single(args):
     import torch
@@ -435,6 +453,8 @@ def run_single(args):
     launches = m.profile_read(reset=True)["launches"]
     s0 += K
     value = pts / (ms_total * 1e-3) / 1e6
+    if args.dump_outputs:
+        dump_outputs(m, args.dump_outputs)
 
     # ---- per-kernel durations: a SERIAL pass (gem_profile_enable makes the add calls issue bin -> fold_long -> fold
     # one after the other on one stream, each bracketed by CUDA events: no overlap, so the figures are uncontended) ----
@@ -683,8 +703,12 @@ def main():
     ap.add_argument("--warmup", type=int, default=20)
     ap.add_argument("--impl", default="gem_b200", choices=["gem_b200", "reference"])
     ap.add_argument("--frames", type=int, default=64, help="distinct synthetic frames cycled (64 x 2.5 MB > L2)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the map the timed steps left behind to DIR/<layer>.npy (--gpus 1 only)")
     args = ap.parse_args()
     world = int(os.environ.get("WORLD_SIZE", "1"))
+    if args.dump_outputs and (args.impl != "gem_b200" or args.gpus > 1 or world > 1):
+        ap.error("--dump-outputs is supported on the single-GPU gem_b200 path only")
     if args.impl == "reference":
         line = run_reference(args)
     elif args.gpus > 1 or world > 1:

@@ -77,9 +77,10 @@ def test_oracle_reproduces_reference_golden(gold):
     o = OracleMap(int(gold["L"]), float(gold["res"]), compat_box_filter=True)
     out = drive(o, gold)
     check_against_reference(out, gold, "oracle")
-    # and the oracle outputs stored next to them are what this build of the oracle produces
+    # and the oracle outputs stored next to them are what this build of the oracle produces (its EXACT outputs were
+    # bit-identical to ref_nofma's when the file was made, so check_against_reference covers them)
     for k in range(int(gold["nframes"])):
-        for name in EXACT + ("feat_traver", "feat_rough", "feat_slope"):
+        for name in ("feat_traver", "feat_rough", "feat_slope"):
             a, b = out[f"f{k}_{name}"], gold[f"oracle_f{k}_{name}"]
             same = (bits(np.asarray(a, b.dtype)) == bits(b)) | (np.isnan(np.asarray(a, np.float64)) & np.isnan(np.asarray(b, np.float64)))
             assert same.all(), f"oracle drifted from its committed output: frame {k} {name}"
